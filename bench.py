@@ -12,9 +12,11 @@ Python API from pinned HOST buffers (H2D of the step's inputs and D2H of the upd
 inside the timed region).  The renderer (2^18-ray batches x 72 samples through the fused
 marcher) is reported in the same line under "render".
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 N > 1: one rank per GPU under torchrun; every rank owns an independent keyframe window and
 ray batch (weak scaling, no data-path collective — SURVEY §8e), time = max over ranks.
+--dump-outputs DIR writes the updated poses / inverse depths and the lookup features of the last
+timed step as DIR/<name>.npy (float32); inputs are seeded, so two builds can be compared on them.
 """
 import argparse
 import json
@@ -422,15 +424,37 @@ def stereo_build_leg(dev, rank, steps, warm, pk):
                                 "unit": "GB/s", "frac": lb / (ms_l * 1e-3) / 1e9 / pk["hbm"], "algorithmic_bytes": lb}}
 
 
-def window_leg(sc, dev, steps, warm, barrier, world, pk, clock_index=None):
-    """device-resident + end-to-end timing of the keyframe-BA-update on one window shape"""
+DUMP_SAMPLE = 1 << 22          # elements kept of a dumped output larger than this (16 MB in float32)
+
+
+def dump_outputs(out_dir, outputs):
+    """out_dir/<name>.npy in float32 for each output; of one with more than DUMP_SAMPLE elements, the elements at a
+    fixed seeded sample of flat indices (ascending), the same for every run with the same arguments"""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in outputs.items():
+        a = t.detach().float().cpu().numpy().reshape(-1)
+        if a.size > DUMP_SAMPLE:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_SAMPLE, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a.reshape(t.shape) if a.size == t.numel() else a)
+
+
+def window_leg(sc, dev, steps, warm, barrier, world, pk, clock_index=None, dump_dir=None):
+    """device-resident + end-to-end timing of the keyframe-BA-update on one window shape; with dump_dir, what the
+    last timed step computed (BA poses and inverse depths, lookup features) is written there"""
     win = Window(sc, dev)
+    last = {}
+
+    def step():
+        last["corr"] = win.step()
+
     if clock_index is not None:
         with ClockSampler(clock_index) as clk:
-            ms_step = time_gpu(win.step, steps, warm, barrier)
+            ms_step = time_gpu(step, steps, warm, barrier)
         clocks = clk.summary()
     else:
-        ms_step, clocks = time_gpu(win.step, steps, warm, barrier), None
+        ms_step, clocks = time_gpu(step, steps, warm, barrier), None
+    if dump_dir is not None:
+        dump_outputs(dump_dir, {"poses": win.d["poses"], "disps": win.d["disps"], "corr": last["corr"]})
     ms_step = max_over_ranks(ms_step, world)
     outp = (torch.empty_like(sc["poses"]).pin_memory(), torch.empty_like(sc["disps"]).pin_memory())
     ms_e2e = max_over_ranks(time_gpu(lambda: win.step_e2e(outp), steps, warm, barrier), world)
@@ -734,6 +758,8 @@ def main():
     ap.add_argument("--no-render", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--only", default="", help="comma list of legs to run besides the main one: headline,sharded,full,render,mapping")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the main leg computed (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -763,7 +789,8 @@ def main():
 
     # ---- configs[1]: the metric's own configuration (value / e2e / roofline of the line)
     sc = make_window(43 + rank)
-    main_rec, clocks = window_leg(sc, dev, args.steps, warm, barrier, world, pk, clock_index=local)
+    main_rec, clocks = window_leg(sc, dev, args.steps, warm, barrier, world, pk, clock_index=local,
+                                  dump_dir=args.dump_outputs if rank == 0 else None)
     line = {"metric": METRIC, "value": main_rec["value"], "unit": "updates/s", "n_gpus": world,
             "steps": args.steps, "warmup": warm, "ms_per_step": main_rec["ms_per_step"], "higher_is_better": True,
             "scaling": "weak", "vs_baseline": None, "dtype": "f16 corr (f32 accumulate) / f32 BA (f64 solve)",

@@ -377,6 +377,8 @@ def gen_render_z():
 def gen_cvx_upsample():
     dn = ref_import("src.droid_net")
     g = torch.Generator().manual_seed(77)
+    # one thread: torch's float16 softmax then rounds the same on every host (see oracle/upsample_oracle.py)
+    torch.set_num_threads(1)
     out = {}
     for tag, (b, ht, wd, dim) in {"disp": (3, 6, 9, 1), "flow": (2, 5, 7, 2)}.items():
         data = torch.rand(b, ht, wd, dim, generator=g) + 0.1
