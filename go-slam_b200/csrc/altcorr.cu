@@ -10,7 +10,7 @@
 // feature vector is staged once per pixel in shared memory; a block covers 32 consecutive
 // pixels and writes the 49 channels with coalesced 128-byte rows.
 #include "common.cuh"
-#include <mutex>
+#include "launch.cuh"
 #include <cstdlib>
 
 namespace {
@@ -331,20 +331,11 @@ altcorr_tc_kernel(const AltPyrArgs a) {
 
 }  // namespace
 
-// opt-in dynamic shared memory is a PER-DEVICE function attribute: one flag per device ordinal, set under a mutex
-static bool altcorr_device_attrs() {
-  static bool ready[64];
-  static std::mutex mu;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64) return false;
-  std::lock_guard<std::mutex> lock(mu);
-  if (ready[dev]) return true;
-  if (cudaFuncSetAttribute(altcorr_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess ||
-      cudaFuncSetAttribute(altcorr_pyramid_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024) != cudaSuccess)
-    return false;
-  ready[dev] = true;
-  return true;
+static GsDeviceOnce g_altcorr_once;
+static cudaError_t altcorr_device_init(int) {
+  cudaError_t e = cudaFuncSetAttribute(altcorr_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(altcorr_pyramid_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
+  return e;
 }
 
 extern "C" {
@@ -358,7 +349,7 @@ int goslam_altcorr_forward(const float* fmap1, const float* fmap2, const float* 
   if (S > 65535 || B > 65535) return GOSLAM_EINVAL;
   const size_t smem = (size_t)(kWarps * C + kWarps * 64 + 49 * (kPixPerBlock + 1)) * sizeof(float);
   if (smem > 200 * 1024) return GOSLAM_EINVAL;
-  if (!altcorr_device_attrs()) return GOSLAM_ELAUNCH;
+  { const int rc = gs_device_once(g_altcorr_once, altcorr_device_init); if (rc != GOSLAM_OK) return rc; }
   dim3 grid(gs_cdiv(H * W, kPixPerBlock), S, B);
   altcorr_kernel<3><<<grid, kWarps * 32, smem, (cudaStream_t)stream>>>(fmap1, fmap2, coords, corr,
                                                                        S, H, W, H2, W2, C);
@@ -384,13 +375,8 @@ int goslam_altcorr_pyramid(const void* const* pyramid, int num_levels, const flo
   a.N = N; a.H = H; a.W = W; a.C = C; a.L = num_levels;
   const size_t smem = (size_t)(kWarps * C + kWarps * 64 + 49 * (kPixPerBlock + 1)) * sizeof(float);
   if (smem > 200 * 1024) return GOSLAM_EINVAL;
-  if (!altcorr_device_attrs()) return GOSLAM_ELAUNCH;
-#ifdef GOSLAM_ALTCORR_FORCE_SIMT     // build-time A/B switch (tools/time_altcorr.py), never in the shipped library
-  constexpr bool force_simt = true;
-#else
-  constexpr bool force_simt = false;
-#endif
-  if (C == 128 && !force_simt) {                   // tensor-core path (the model's feature width)
+  { const int rc = gs_device_once(g_altcorr_once, altcorr_device_init); if (rc != GOSLAM_OK) return rc; }
+  if (C == 128) {                   // tensor-core path (the model's feature width)
     dim3 grid(gs_cdiv(H * W, kTcPix), N, num_levels);
     altcorr_tc_kernel<3><<<grid, kTcWarps * 32, 0, (cudaStream_t)stream>>>(a);
   } else {

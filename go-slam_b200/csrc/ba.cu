@@ -31,11 +31,11 @@
 // zeroed (:320-323); stereo baseline (-0.1,0,0) (:219-229); MIN_DEPTH 0.25 (:26);
 // damping diag += ep + lm*diag (:1197); failed factorisation => dx = 0 (:1207-1210).
 #include "common.cuh"
+#include "launch.cuh"
 #include <cstring>
 #include "se3.cuh"
 #include <algorithm>
 #include <cstdio>
-#include <mutex>
 #include <cooperative_groups.h>
 
 namespace {
@@ -1544,51 +1544,30 @@ bool make_dims(int N, int num, int ht, int wd, int t0, int t1, BaDims* d) {
 
 constexpr int kSmemSolveMaxN = 160;   // (160*160 + 160) * 8 B = 206 KB of the 227 KB
 constexpr int kWarpSolveMaxN = 96;    // single-warp solve up to 16 poses
-constexpr int kMaxDevices = 64;
 constexpr size_t kClusterSmemMax = 226 * 1024;   // dynamic part of the 227 KB per-CTA opt-in maximum (static: a few bytes)
-
-// Function attributes (opt-in dynamic shared memory) and the occupancy of the cooperative kernel
-// are PER DEVICE: a process that runs BA on a second GPU must set them there too.  One slot per
-// device ordinal, initialised once under a mutex (the C-ABI may be called from several threads).
-struct BaDevice {
-  bool ready = false;
-  int sms = 0;
-  int blocks_per_sm = 0;      // 0: cooperative launch unavailable -> multi-kernel driver
-};
-
-void ba_persistent_kernel_attrs(BaDevice* dv, int dev) {
-  int occ = 0, coop = 0;
-  const size_t smem_max = ((size_t)kWarpSolveMaxN * kWarpSolveMaxN + 2 * kWarpSolveMaxN) * sizeof(double);
-  cudaDeviceGetAttribute(&dv->sms, cudaDevAttrMultiProcessorCount, dev);
-  cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
-  cudaFuncSetAttribute(ba_persistent_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem_max);
-  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ba_persistent_kernel, kTP, smem_max);
-  constexpr int kWant = 2;    // 2 blocks/SM measured best (profiles/r01: 1 -> 151 us, 2 -> 121 us, 3 -> 124 us)
-  dv->blocks_per_sm = (!coop || occ < 1) ? 0 : (occ > kWant ? kWant : occ);
-}
 
 inline size_t prep_smem_bytes(int num) { return ((size_t)3 * num + 1 + 33) * sizeof(int); }
 
-const BaDevice& ba_device() {
-  static BaDevice table[kMaxDevices];
-  static std::mutex mu;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= kMaxDevices) dev = 0;
-  std::lock_guard<std::mutex> lock(mu);
-  BaDevice& dv = table[dev];
-  if (!dv.ready) {
-    cudaFuncSetAttribute(ba_prep_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)prep_smem_bytes(kPrepMaxFrames));
-    cudaFuncSetAttribute(ba_solve_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         (int)(((size_t)kSmemSolveMaxN * kSmemSolveMaxN + kSmemSolveMaxN) * 8));
-    cudaFuncSetAttribute(ba_solve_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         (int)(((size_t)kWarpSolveMaxN * kWarpSolveMaxN + 2 * kWarpSolveMaxN) * 8));
-    cudaFuncSetAttribute(ba_solve_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                         (int)kClusterSmemMax);
-    ba_persistent_kernel_attrs(&dv, dev);
-    dv.ready = true;
-  }
-  return dv;
+// Function attributes (opt-in dynamic shared memory) and the occupancy of the cooperative kernel are PER DEVICE.
+GsDeviceOnce g_ba_once;
+int g_blocks_per_sm[kGsMaxDevices];     // 0: cooperative launch unavailable -> multi-kernel driver
+
+cudaError_t ba_device_init(int dev) {
+  const size_t smem_max = ((size_t)kWarpSolveMaxN * kWarpSolveMaxN + 2 * kWarpSolveMaxN) * sizeof(double);
+  constexpr cudaFuncAttribute kSmem = cudaFuncAttributeMaxDynamicSharedMemorySize;
+  cudaError_t e = cudaFuncSetAttribute(ba_prep_kernel, kSmem, (int)prep_smem_bytes(kPrepMaxFrames));
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(ba_solve_kernel, kSmem, (int)(((size_t)kSmemSolveMaxN * kSmemSolveMaxN + kSmemSolveMaxN) * 8));
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(ba_solve_warp_kernel, kSmem, (int)smem_max);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(ba_solve_cluster_kernel, kSmem, (int)kClusterSmemMax);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(ba_persistent_kernel, kSmem, (int)smem_max);
+  if (e != cudaSuccess) return e;
+  int occ = 0, coop = 0;
+  cudaDeviceGetAttribute(&coop, cudaDevAttrCooperativeLaunch, dev);
+  cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, ba_persistent_kernel, kTP, smem_max);
+  constexpr int kWant = 2;    // 2 blocks/SM measured best (profiles/r01: 1 -> 151 us, 2 -> 121 us, 3 -> 124 us)
+  g_blocks_per_sm[dev] = (!coop || occ < 1) ? 0 : (occ > kWant ? kWant : occ);
+  return cudaSuccess;
 }
 
 
@@ -1620,8 +1599,7 @@ int launch_phase2(float* poses, float* disps, const SysSrc& sys_in,
                   const BaDims& d, const BaWs& ws, float lm, float ep, int motion_only,
                   int owner_lo, int owner_hi, float* dx_out, float* dz_out, int* status_out,
                   cudaStream_t st, const PeerRows& peer_rows = PeerRows{}) {
-  const BaDevice& dv = ba_device();    // per-device function attributes are set on first use
-  (void)dv;
+  { const int rc = gs_device_once(g_ba_once, ba_device_init); if (rc != GOSLAM_OK) return rc; }
   if (d.n <= kWarpSolveMaxN) {
     const size_t smem = ((size_t)d.n * d.n + 2 * d.n) * sizeof(double);
     ba_solve_warp_kernel<<<1, 128, smem, st>>>(poses, d, ws, sys_in, lm, ep, dx_out, status_out);
@@ -1686,14 +1664,11 @@ int goslam_ba(float* poses, float* disps, const float* intrinsics, const float* 
   const size_t need = ba_layout(d, workspace, workspace_bytes, &ws);
   if (workspace == nullptr || need > workspace_bytes) return GOSLAM_EWORKSPACE;
   cudaStream_t st = (cudaStream_t)stream;
-#ifdef GOSLAM_BA_FORCE_MULTIKERNEL      // build-time A/B switch (tools/), never in the shipped library
-  constexpr bool multi_kernel = true;
-#else
-  constexpr bool multi_kernel = false;
-#endif
-  if (d.n <= kWarpSolveMaxN && !multi_kernel) {
-    const BaDevice& dv = ba_device();
-    const int blocks_per_sm = dv.blocks_per_sm, sms = dv.sms;
+  if (d.n <= kWarpSolveMaxN) {
+    { const int rc = gs_device_once(g_ba_once, ba_device_init); if (rc != GOSLAM_OK) return rc; }
+    int dev = 0;
+    cudaGetDevice(&dev);
+    const int blocks_per_sm = g_blocks_per_sm[dev], sms = gs_sm_count();
     const size_t smem = ((size_t)d.n * d.n + 2 * d.n) * sizeof(double);
     if (blocks_per_sm > 0) {
       // two launches per call: the table kernel (which also zeroes the reduced system and the barrier

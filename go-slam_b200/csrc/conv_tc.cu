@@ -26,8 +26,8 @@
 // fp16 operands, fp32 accumulation, fp32 gate arithmetic, fp16 state — what the reference's autocast region
 // computes (src/factor_graph.py:198, torch.cuda.amp.autocast) with one rounding less per gate.
 #include "common.cuh"
+#include "launch.cuh"
 #include "tc_ptx.cuh"
-#include <mutex>
 
 using namespace gs_tc;
 
@@ -667,100 +667,53 @@ scatter_mean_kernel(const __half* __restrict__ a1, const int* __restrict__ slot,
   *reinterpret_cast<uint4*>(mean + ((size_t)m * hw + px) * 128 + c8 * 8) = *reinterpret_cast<const uint4*>(o);
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn conv_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn) return fn;
-  void* ptr = nullptr;
-  cudaDriverEntryPointQueryResult q;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &ptr, cudaEnableDefault, &q) != cudaSuccess ||
-      q != cudaDriverEntryPointSuccess)
-    return nullptr;
-  fn = reinterpret_cast<EncodeTiledFn>(ptr);
-  return fn;
-}
-
 // Tensor maps depend only on (base pointer, shape): the update operator runs the same layers on the same workspace
-// buffers call after call, so the driver's encode (~1.5 us of host time each, ~50 per operator call) is cached.
-struct CMapKey { const void* base; int a, b, c, d, kind; };
-struct CMapSlot { CMapKey key; CUtensorMap map; unsigned long long stamp; bool used; };
-constexpr int kCMapSlots = 128;
-bool act_map_raw(EncodeTiledFn enc, const void* base, int B, int h, int w, int C, CUtensorMap* out);
-bool weight_map_raw(EncodeTiledFn enc, const void* base, int taps, int N, int Cin, CUtensorMap* out, int n_tile);
+// buffers call after call, so the encodes (~50 per operator call) are paid once.
+enum { kActMap = 0, kWeightMap = 1 };
 
-bool cached_cmap(EncodeTiledFn enc, const CMapKey& k, CUtensorMap* out) {
-  static CMapSlot table[kCMapSlots];
-  static unsigned long long clock = 0;
-  static std::mutex mu;
-  std::lock_guard<std::mutex> lock(mu);
-  int victim = -1;
-  for (int i = 0; i < kCMapSlots; ++i) {
-    CMapSlot& s = table[i];
-    if (s.used && s.key.base == k.base && s.key.a == k.a && s.key.b == k.b && s.key.c == k.c && s.key.d == k.d &&
-        s.key.kind == k.kind) {
-      s.stamp = ++clock;
-      *out = s.map;
-      return true;
-    }
-    if (victim < 0 || (table[victim].used && (!s.used || s.stamp < table[victim].stamp))) victim = i;
+bool encode_cmap(GsEncodeTiledFn enc, const GsMapKey& k, CUtensorMap* out) {
+  if (k.kind == kActMap) {
+    // activation map: NHWC [B, h, w, C] as (ch, x, y, image), box 64 ch x 16 x 8
+    const int B = k.dims[0], h = k.dims[1], w = k.dims[2], C = k.dims[3];
+    cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)B};
+    cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)w * C * 2, (cuuint64_t)h * w * C * 2};
+    cuuint32_t box[4] = {(cuuint32_t)kKC, (cuuint32_t)kPX, (cuuint32_t)kPY, 1};
+    cuuint32_t es[4] = {1, 1, 1, 1};
+    return enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(k.base), dims, strides, box, es,
+               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
+               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
   }
-  CMapSlot& v = table[victim];
-  const bool ok = k.kind == 0 ? act_map_raw(enc, k.base, k.a, k.b, k.c, k.d, &v.map)
-                              : weight_map_raw(enc, k.base, k.a, k.b, k.c, &v.map, k.d);
-  if (!ok) { v.used = false; return false; }
-  v.key = k; v.used = true; v.stamp = ++clock;
-  *out = v.map;
-  return true;
-}
-bool act_map(EncodeTiledFn enc, const void* base, int B, int h, int w, int C, CUtensorMap* out) {
-  return cached_cmap(enc, CMapKey{base, B, h, w, C, 0}, out);
-}
-bool weight_map(EncodeTiledFn enc, const void* base, int taps, int N, int Cin, CUtensorMap* out, int n_tile = 0) {
-  return cached_cmap(enc, CMapKey{base, taps, N, Cin, n_tile, 1}, out);
-}
-
-// activation map: NHWC [B, h, w, C] as (ch, x, y, image), box 64 ch x 16 x 8
-bool act_map_raw(EncodeTiledFn enc, const void* base, int B, int h, int w, int C, CUtensorMap* out) {
-  cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)B};
-  cuuint64_t strides[3] = {(cuuint64_t)C * 2, (cuuint64_t)w * C * 2, (cuuint64_t)h * w * C * 2};
-  cuuint32_t box[4] = {(cuuint32_t)kKC, (cuuint32_t)kPX, (cuuint32_t)kPY, 1};
-  cuuint32_t es[4] = {1, 1, 1, 1};
-  return enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(base), dims, strides, box, es,
-             CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-             CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-}
-// weight map: [taps, N, Cin] as (cin, cout, tap), box 64 x N
-bool weight_map_raw(EncodeTiledFn enc, const void* base, int taps, int N, int Cin, CUtensorMap* out, int n_tile) {
+  // weight map: [taps, N, Cin] as (cin, cout, tap), box 64 x n_tile (0: N)
+  const int taps = k.dims[0], N = k.dims[1], Cin = k.dims[2], n_tile = k.dims[3];
   cuuint64_t dims[3] = {(cuuint64_t)Cin, (cuuint64_t)N, (cuuint64_t)taps};
   cuuint64_t strides[2] = {(cuuint64_t)Cin * 2, (cuuint64_t)N * Cin * 2};
   cuuint32_t box[3] = {(cuuint32_t)kKC, (cuuint32_t)(n_tile > 0 ? n_tile : N), 1};
   cuuint32_t es[3] = {1, 1, 1};
-  return enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(base), dims, strides, box, es,
+  return enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 3, const_cast<void*>(k.base), dims, strides, box, es,
              CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
+GsMapCache g_cmaps(128, encode_cmap);
+
+bool act_map(const void* base, int B, int h, int w, int C, CUtensorMap* out) {
+  return g_cmaps.get(GsMapKey{base, kActMap, {B, h, w, C}}, out);
+}
+bool weight_map(const void* base, int taps, int N, int Cin, CUtensorMap* out, int n_tile = 0) {
+  return g_cmaps.get(GsMapKey{base, kWeightMap, {taps, N, Cin, n_tile}}, out);
+}
+
+GsDeviceOnce g_conv_once;
+cudaError_t conv_device_init(int) {
+  cudaError_t e = cudaFuncSetAttribute(conv_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemC);
+  if (e == cudaSuccess) e = cudaFuncSetAttribute(flow7x7_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kF7Smem);
+  return e;
+}
+
 int conv_launch(const ConvMaps& maps, ConvParams p, cudaStream_t st) {
-  static int sm_count[64];
-  static std::mutex mu;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64) dev = 0;
-  int sms;
-  {
-    std::lock_guard<std::mutex> lock(mu);
-    if (sm_count[dev] == 0) {
-      if (cudaFuncSetAttribute(conv_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemC) != cudaSuccess)
-        return GOSLAM_ELAUNCH;
-      int n = 148;
-      cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-      sm_count[dev] = n > 0 ? n : 148;
-    }
-    sms = sm_count[dev];
-  }
+  const int rc = gs_device_once(g_conv_once, conv_device_init);
+  if (rc != GOSLAM_OK) return rc;
+  const int sms = gs_sm_count();
   p.n_yb = gs_cdiv(p.h, kPY); p.n_xb = gs_cdiv(p.w, kPX);
   if (p.n_nt < 1) p.n_nt = 1;
   p.n_tiles = p.B * p.n_yb * p.n_xb * p.n_nt;
@@ -829,8 +782,6 @@ int goslam_conv2d_nhwc(const goslam_conv_desc* d, int B, int h, int w, void* str
   const int N = d->cout_pad <= kMaxN ? d->cout_pad : (d->cout_pad % 192 == 0 ? 192 : (d->cout_pad % 256 == 0 ? 256 : 128));
   if (d->cout_pad % N) return GOSLAM_EINVAL;
   if (B == 0) return GOSLAM_OK;
-  EncodeTiledFn enc = conv_encode_fn();
-  if (!enc) return GOSLAM_ELAUNCH;
   ConvMaps m{};
   ConvParams p{};
   p.B = B; p.h = h; p.w = w; p.taps = d->taps; p.n_in = d->n_in; p.N = N; p.n_nt = d->cout_pad / N;
@@ -839,9 +790,9 @@ int goslam_conv2d_nhwc(const goslam_conv_desc* d, int B, int h, int w, void* str
     if (d->cin[i] <= 0 || d->cin[i] % kKC || d->cin_off[i] % kKC || d->cin_stride[i] < d->cin_off[i] + d->cin[i]) return GOSLAM_EINVAL;
     p.chunks[i] = d->cin[i] / kKC; p.coff[i] = d->cin_off[i];
     cin_total += d->cin[i];
-    if (!act_map(enc, d->in[i], B, h, w, d->cin_stride[i], &m.in[i])) return GOSLAM_ELAUNCH;
+    if (!act_map(d->in[i], B, h, w, d->cin_stride[i], &m.in[i])) return GOSLAM_ELAUNCH;
   }
-  if (!weight_map(enc, d->weight, d->taps, d->cout_pad, cin_total, &m.w, N)) return GOSLAM_ELAUNCH;
+  if (!weight_map(d->weight, d->taps, d->cout_pad, cin_total, &m.w, N)) return GOSLAM_ELAUNCH;
   p.epi = EPI_ACT; p.bias = d->bias; p.act = d->act; p.cout = d->cout; p.out = d->out; p.out_f32 = d->out_f32;
   p.out_stride = d->out_stride; p.out_offset = d->out_offset; p.out_scale = d->out_scale;
   p.split = d->split; p.act2 = d->act2; p.out2 = d->out2;
@@ -931,26 +882,10 @@ int goslam_update_op(const goslam_update_weights* W, const void* net, const void
   GS_TRY(layer(ws.c1, 128, 0, 128, W->corr2_w, W->corr2_b, 9, 128, 128, ACT_RELU, 1.f, ws.c2, 0, 128, N, h, w, stream));
   {
     // 7x7 motion encoder: im2col + tcgen05 (flow0_w f16 [128][256], K = (ky*7+kx)*4 + ci, zero beyond 196)
-    EncodeTiledFn enc = conv_encode_fn();
     CUtensorMap wm;
-    if (!enc || !weight_map(enc, W->flow0_w, 1, 128, kF7K, &wm, 128)) return GOSLAM_ELAUNCH;
-    static int sm_count[64];
-    static std::mutex mu;
-    int dev = 0;
-    cudaGetDevice(&dev);
-    if (dev < 0 || dev >= 64) dev = 0;
-    int sms;
-    {
-      std::lock_guard<std::mutex> lock(mu);
-      if (sm_count[dev] == 0) {
-        if (cudaFuncSetAttribute(flow7x7_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kF7Smem) != cudaSuccess)
-          return GOSLAM_ELAUNCH;
-        int n = 148;
-        cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-        sm_count[dev] = n > 0 ? n : 148;
-      }
-      sms = sm_count[dev];
-    }
+    if (!weight_map(W->flow0_w, 1, 128, kF7K, &wm, 128)) return GOSLAM_ELAUNCH;
+    GS_TRY(gs_device_once(g_conv_once, conv_device_init));
+    const int sms = gs_sm_count();
     const int n_tiles = N * gs_cdiv(h, kPY) * gs_cdiv(w, kPX);
     flow7x7_tc_kernel<<<n_tiles < sms ? n_tiles : sms, 160, kF7Smem, st>>>(wm, flow, W->flow0_b, ws.f1, N, h, w);
     GS_CHECK_LAUNCH();
@@ -994,15 +929,13 @@ int goslam_conv_gru(const goslam_gru_weights* wts, const void* net, const void* 
   GruWs ws;
   const size_t need = gru_layout(B, h, w, workspace, workspace_bytes, &ws);
   if (workspace == nullptr || need > workspace_bytes) return GOSLAM_EWORKSPACE;
-  EncodeTiledFn enc = conv_encode_fn();
-  if (!enc) return GOSLAM_ELAUNCH;
   cudaStream_t st = (cudaStream_t)stream;
   ConvMaps m{};
   ConvParams p{};
   p.B = B; p.h = h; p.w = w;
   p.net = reinterpret_cast<const __half*>(net);
   // ---- pass G: glo_sum = sum_px sigmoid(w(net)) * net
-  if (!act_map(enc, net, B, h, w, 128, &m.in[0]) || !weight_map(enc, wts->w_w, 1, 128, 128, &m.w)) return GOSLAM_ELAUNCH;
+  if (!act_map(net, B, h, w, 128, &m.in[0]) || !weight_map(wts->w_w, 1, 128, 128, &m.w)) return GOSLAM_ELAUNCH;
   p.n_nt = 1;
   p.taps = 1; p.n_in = 1; p.chunks[0] = 2; p.N = 128; p.epi = EPI_GLO; p.bias = wts->b_w; p.glo = nullptr;
   p.glo_sum = ws.glo_sum;
@@ -1012,15 +945,15 @@ int goslam_conv_gru(const goslam_gru_weights* wts, const void* net, const void* 
                                        1.0f / (float)(h * w));
   GS_CHECK_LAUNCH();
   // ---- pass ZR: z, r*net
-  if (!act_map(enc, inp, B, h, w, 128, &m.in[1]) || !act_map(enc, corr, B, h, w, 128, &m.in[2]) ||
-      !act_map(enc, flow, B, h, w, 64, &m.in[3]) || !weight_map(enc, wts->w_zr, 9, 256, 448, &m.w))
+  if (!act_map(inp, B, h, w, 128, &m.in[1]) || !act_map(corr, B, h, w, 128, &m.in[2]) ||
+      !act_map(flow, B, h, w, 64, &m.in[3]) || !weight_map(wts->w_zr, 9, 256, 448, &m.w))
     return GOSLAM_ELAUNCH;
   p.taps = 9; p.n_in = 4; p.chunks[0] = 2; p.chunks[1] = 2; p.chunks[2] = 2; p.chunks[3] = 1;
   p.N = 256; p.epi = EPI_ZR; p.bias = wts->b_zr; p.glo = ws.glo; p.z_out = ws.z; p.rnet_out = ws.rnet;
   rc = conv_launch(m, p, st);
   if (rc) return rc;
   // ---- pass Q: net' = (1 - z) net + z tanh(convq([r*net | inp | corr | flow]) + glo_q)
-  if (!act_map(enc, ws.rnet, B, h, w, 128, &m.in[0]) || !weight_map(enc, wts->w_q, 9, 128, 448, &m.w)) return GOSLAM_ELAUNCH;
+  if (!act_map(ws.rnet, B, h, w, 128, &m.in[0]) || !weight_map(wts->w_q, 9, 128, 448, &m.w)) return GOSLAM_ELAUNCH;
   p.N = 128; p.epi = EPI_Q; p.bias = wts->b_q; p.z_in = ws.z; p.net_out = reinterpret_cast<__half*>(net_out);
   return conv_launch(m, p, st);
 }

@@ -26,12 +26,9 @@
 // The 1/4 feature scaling of the reference (`fmap / 4.0` in half) is applied by the K-major
 // re-layout prepass, exactly as the reference does it, so the accumulator needs no scaling.
 #include "common.cuh"
+#include "launch.cuh"
 #include "tc_ptx.cuh"
-#include <mutex>
 #include <cstdio>
-#include <cuda.h>
-#include <cstdlib>
-#include <cstring>
 
 int gs_corr_build_simt_f16(const __half* f1, const __half* f2, __half* const* levels,
                            int num_levels, int N, int D, int h, int w, cudaStream_t st);
@@ -50,7 +47,7 @@ constexpr int kEpiWarps = 8;                      // per group (2 per TMEM lane 
 constexpr int kEpiThreads = kTStages * kEpiWarps * 32;   // 512
 constexpr int kThreadsTC = 64 + kEpiThreads;             // 576
 constexpr int kMaxXB = 8;                                // x-tiles per band (w <= 128)
-constexpr int kPoolMax = kBM * ((4 * kMaxXB * 16 + 16) + (2 * kMaxXB * 8 + 48));  // 90,112 B (level 1 | level 2 + 3 pieces)
+constexpr int kPoolMax = kBM * ((4 * kMaxXB * 16 + 16) + (2 * kMaxXB * 8 + 8));   // 84,992 B (level 1 | level 2 pieces)
 constexpr int kSmemTC = 1024 + (kAStages + kBStages) * kTileBytes + kPoolMax + 256;
 
 using namespace gs_tc;
@@ -73,9 +70,6 @@ struct TcParams {
   int tiled, w4_0, h4_0, w4_1, h4_1;
   int pitch2, pitch3;         // tiled: bytes per (source pixel, band) of levels 2 / 3 (multiples of 32)
   int aligned;                // w % 16 == 0 && h % 8 == 0: every store is a whole aligned sector run
-  int experiment;             // profiling only: 1 = no output writes
-  int bulk;                   // tiled: pooled levels leave through bulk (TMA) stores, asynchronously
-  int pingpong;               // tiled: the two epilogue groups take turns in their level-0 store sections
 };
 
 // ---- packed fp16 rows live in registers as uint32 pairs (lo = even column) ----
@@ -236,15 +230,12 @@ corr_build_tc_kernel(const __grid_constant__ CUtensorMap mapA,
     const int ts = group;
     // band staging strides (bytes); the +16 / +8 pads make the per-source-pixel stride conflict-free
     const int p1row = p.n_xb * 16, p1src = 4 * p1row + 16;
-    const int p2row = p.n_xb * 8;   // (bulk mode keeps the level-3 piece behind the level-2 piece)
-    const int p2src = p.tiled ? p.pitch2 + (p.bulk ? 48 : 8) : 2 * p2row + 8;
+    const int p2row = p.n_xb * 8;
+    const int p2src = p.tiled ? p.pitch2 + 8 : 2 * p2row + 8;
     unsigned char* pool1 = smPool;
     unsigned char* pool2 = smPool + kBM * p1src;
     const int h1 = p.h >> 1, w1 = p.w >> 1, h2 = p.h >> 2, w2 = p.w >> 2, h3 = p.h >> 3, w3 = p.w >> 3;
-    const bool wr = p.experiment != 1;
     int tph = 0, tile = 0;
-    // ordered store sections (ping-pong): named barrier 4+g = "group g may store"; 256 waiters + 256 arrivers
-    if (p.pingpong && group == 1) asm volatile("bar.arrive 4, 512;" ::: "memory");
 #ifdef GOSLAM_TC_PROBE
     long long pr_wait = 0, pr_tiles = 0, pr_bar1 = 0, pr_wo = 0, pr_bar2 = 0, pr_t0 = clock64();
     const bool pr_on = (etid == 0 || etid == 256) && blockIdx.x == 0;
@@ -258,7 +249,7 @@ corr_build_tc_kernel(const __grid_constant__ CUtensorMap mapA,
       const int mt = (item / p.n_yb) % p.n_mt;
       const int n = item / (p.n_yb * p.n_mt);
       const int src = mt * kBM + row;
-      const bool src_ok = src < p.hw && wr;
+      const bool src_ok = src < p.hw;
       const int n_out = p.out_slot ? __ldg(p.out_slot + n) : n;
       const long long plane_id = (long long)n_out * p.hw + src;
       const int y0 = yb * kPY;
@@ -293,10 +284,6 @@ corr_build_tc_kernel(const __grid_constant__ CUtensorMap mapA,
           __syncwarp();
           if (lane == 0) mbar_arrive(&tm_empty[ts]);
           const int ty = 2 * yb + half;
-          if (p.pingpong) {
-            if (group == 0) asm volatile("bar.sync 4, 512;" ::: "memory");
-            else asm volatile("bar.sync 5, 512;" ::: "memory");
-          }
           if (src_ok && ty < p.h4_0) {
             unsigned char* dst = reinterpret_cast<unsigned char*>(p.lvl[0]) +
                                  ((plane_id * p.h4_0 + ty) * p.w4_0 + xb * 4) * 32LL;
@@ -307,10 +294,6 @@ corr_build_tc_kernel(const __grid_constant__ CUtensorMap mapA,
                              "r"(hr[0][2 * t]), "r"(hr[0][2 * t + 1]), "r"(hr[1][2 * t]), "r"(hr[1][2 * t + 1]),
                              "r"(hr[2][2 * t]), "r"(hr[2][2 * t + 1]), "r"(hr[3][2 * t]), "r"(hr[3][2 * t + 1])
                              : "memory");
-          }
-          if (p.pingpong) {                          // the other group's turn
-            if (group == 0) asm volatile("bar.arrive 5, 512;" ::: "memory");
-            else asm volatile("bar.arrive 4, 512;" ::: "memory");
           }
 #pragma unroll
           for (int cc = 0; cc < 2; ++cc) {
@@ -366,46 +349,16 @@ corr_build_tc_kernel(const __grid_constant__ CUtensorMap mapA,
       }
       // ---- band write-out: all 16 epilogue warps have staged every x-tile of this 8-row band ----
       TCP(const long long tb = clock64(); pr_tiles += tb - ta;)
-      if (p.bulk) fence_async_smem();            // staged rows become visible to the async (TMA) proxy
       asm volatile("bar.sync 3, 512;" ::: "memory");
       TCP(const long long tc = clock64(); pr_bar1 += tc - tb;)
-      if (wr && p.num_levels > 1) {
+      if (p.num_levels > 1) {
         const int s_loc = etid >> 2, part = etid & 3;          // four threads per source pixel
         const int s_glb = mt * kBM + s_loc;
         if (s_glb < p.hw) {
           const long long pl = (long long)n_out * p.hw + s_glb;
           const unsigned char* sp1 = pool1 + s_loc * p1src;
           const unsigned char* sp2 = pool2 + s_loc * p2src;
-          if (p.tiled && p.bulk) {
-            // The staged pieces are byte-for-byte what goes to memory: hand them to the TMA engine
-            // (one bulk copy per source pixel and level) and go back to draining accumulators; the
-            // copies stream out while the next band's level-0 stores are being issued.
-            if (part == 0 && yb < p.h4_1)
-              bulk_store(reinterpret_cast<unsigned char*>(p.lvl[1]) + ((pl * p.h4_1 + yb) * p.w4_1) * 32LL, sp1,
-                         (uint32_t)p.w4_1 * 32u);
-            if (part == 1 && p.num_levels > 2 && 2 * yb < h2)
-              bulk_store(reinterpret_cast<unsigned char*>(p.lvl[2]) + (pl * p.n_yb + yb) * (long long)p.pitch2, sp2,
-                         (uint32_t)p.pitch2);
-            if (part == 2 && p.num_levels > 3 && yb < h3) {
-              uint32_t* s3 = reinterpret_cast<uint32_t*>(const_cast<unsigned char*>(sp2) + p.pitch2);
-#pragma unroll
-              for (int k = 0; k < 8; ++k) {
-                uint32_t v = 0u;
-                if (k < p.n_xb) {
-                  const uint32_t t = *reinterpret_cast<const uint32_t*>(sp2 + 8 * k);
-                  const uint32_t t2 = *reinterpret_cast<const uint32_t*>(sp2 + 8 * k + 4);
-                  const uint32_t b = *reinterpret_cast<const uint32_t*>(sp2 + p2row + 8 * k);
-                  const uint32_t b2 = *reinterpret_cast<const uint32_t*>(sp2 + p2row + 8 * k + 4);
-                  v = pack2(pool_pair(t, b), pool_pair(t2, b2));
-                }
-                s3[k] = v;
-              }
-              fence_async_smem();
-              bulk_store(reinterpret_cast<unsigned char*>(p.lvl[3]) + (pl * p.n_yb + yb) * 32LL, s3, 32u);
-            }
-            bulk_commit();
-            bulk_wait_read();                      // the staging rows may be overwritten after the next barrier
-          } else if (p.tiled) {
+          if (p.tiled) {
             // level 1: one tile-row of 4x4 tiles = w4_1 contiguous sectors, already in tile order
             if (yb < p.h4_1) {
               unsigned char* g1 = reinterpret_cast<unsigned char*>(p.lvl[1]) +
@@ -449,9 +402,7 @@ corr_build_tc_kernel(const __grid_constant__ CUtensorMap mapA,
                            "r"(rr[1]), "r"(rr[2]), "r"(rr[3]), "r"(rr[4]), "r"(rr[5]), "r"(rr[6]), "r"(rr[7])
                            : "memory");
             }
-          } else
-          if (p.aligned) {
-            if (!p.tiled) {
+          } else if (p.aligned) {
             // level 1: 4 full rows, contiguous in memory, 32-byte aligned: whole sectors
             unsigned char* g1 = reinterpret_cast<unsigned char*>(p.lvl[1]) +
                                 (pl * h1 + (y0 >> 1)) * (long long)p1row;
@@ -462,7 +413,6 @@ corr_build_tc_kernel(const __grid_constant__ CUtensorMap mapA,
               asm volatile("st.global.v8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};" ::"l"(g1 + off), "r"(rr[0]),
                            "r"(rr[1]), "r"(rr[2]), "r"(rr[3]), "r"(rr[4]), "r"(rr[5]), "r"(rr[6]), "r"(rr[7])
                            : "memory");
-            }
             }
             if (part == 1 && p.num_levels > 2) {                // level 2: 2 rows, 16-byte chunks
               unsigned char* g2 = reinterpret_cast<unsigned char*>(p.lvl[2]) +
@@ -486,13 +436,12 @@ corr_build_tc_kernel(const __grid_constant__ CUtensorMap mapA,
             // ragged shapes: element-wise with bounds (staging rows are n_xb*8 / n_xb*4 halves wide)
             const __half* s1 = reinterpret_cast<const __half*>(sp1);
             const __half* s2 = reinterpret_cast<const __half*>(sp2);
-            if (!p.tiled)
-              for (int r = 0; r < 4; ++r) {
-                const int y = (y0 >> 1) + r;
-                if (y >= h1) break;
-                __half* g = p.lvl[1] + (pl * h1 + y) * w1;
-                for (int x = part; x < w1; x += 4) g[x] = s1[r * (p1row / 2) + x];
-              }
+            for (int r = 0; r < 4; ++r) {
+              const int y = (y0 >> 1) + r;
+              if (y >= h1) break;
+              __half* g = p.lvl[1] + (pl * h1 + y) * w1;
+              for (int x = part; x < w1; x += 4) g[x] = s1[r * (p1row / 2) + x];
+            }
             if (p.num_levels > 2)
               for (int r = 0; r < 2; ++r) {
                 const int y = (y0 >> 2) + r;
@@ -517,7 +466,6 @@ corr_build_tc_kernel(const __grid_constant__ CUtensorMap mapA,
       asm volatile("bar.sync 3, 512;" ::: "memory");
       TCP(pr_bar2 += clock64() - td;)
     }
-    if (p.bulk) bulk_wait_all();
 #ifdef GOSLAM_TC_PROBE
     if (pr_on)
       printf("[tc probe etid=%d] total %lld | tile loop %lld (of which tm_full wait %lld) | bar1 %lld | write-out %lld | bar2 %lld\n",
@@ -541,9 +489,6 @@ corr_build_tc_kernel(const __grid_constant__ CUtensorMap mapA,
 // instead of draining accumulators, ends at (no-write floor 116 µs) + (pure-store time 150 µs) = 283 µs.
 // 448 threads: no register cap below the direct-store kernel's 90.
 // ------------------------------------------------------------------------------------------------------
-#ifndef GOSLAM_ST_EXP
-#define GOSLAM_ST_EXP 0          // A/B builds only (tools/build_variant.py): 1 no global stores, 2 no pooling, 4 no level-0 staging
-#endif
 constexpr int kDrainWarps = 8, kStoreWarps = 4;
 constexpr int kThreadsST = 64 + (kDrainWarps + kStoreWarps) * 32;      // 448
 constexpr int kStageRow = 2 * 128 + 16;                                // staged level-0 bytes per source pixel and tile
@@ -551,13 +496,9 @@ constexpr int kStageBytes = kBM * kStageRow;                           // 34,816
 inline int pool_bytes_st(int n_xb) { return kBM * ((4 * n_xb * 16 + 16) + (((n_xb * 16 + 31) / 32 * 32) + 8)); }
 inline int smem_staged(int n_xb) { return 1024 + (1 + kBStages) * kTileBytes + pool_bytes_st(n_xb) + kTStages * kStageBytes + 256; }
 
-// TMA_ST: level 0 leaves the slot as two tensor-map stores per tile (box = 128 source pixels x one 128-byte run, 128-byte
-// swizzle in shared memory) issued by one drain thread; no thread touches the load/store unit for it and the slot is free
-// again as soon as the copy engine has READ it.  The store warps then only write the pooled levels at the end of a band.
-template <int MODE>          // 0: store warps, 1: tensor-map stores, 2: TMEM stage 0 by tensor-map stores, stage 1 by the store warps
 __global__ void __launch_bounds__(kThreadsST, 1)
 corr_build_tc_staged_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant__ CUtensorMap mapB,
-                            const __grid_constant__ CUtensorMap mapO, const TcParams p, const int pool_bytes) {
+                            const TcParams p, const int pool_bytes) {
   extern __shared__ unsigned char smem_raw[];
   unsigned char* base =
       reinterpret_cast<unsigned char*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -661,7 +602,6 @@ corr_build_tc_staged_kernel(const __grid_constant__ CUtensorMap mapA, const __gr
     const int ts = (warp - 2) >> 2;               // TMEM stage = staging slot of this warp
     const int quad = warp & 3;                    // TMEM lane quadrant a warp may read = warp_id % 4
     const int row = quad * 32 + lane;             // source pixel of the tile
-    const bool TMA_ST = MODE == 1 || (MODE == 2 && ts == 0);
     unsigned char* slot = smStage + ts * kStageBytes + row * kStageRow;
     int tph = 0, sph = 0, tile = 0, band = 0;
     for (int item = blockIdx.x; item < p.n_items; item += gridDim.x, ++band) {
@@ -671,12 +611,7 @@ corr_build_tc_staged_kernel(const __grid_constant__ CUtensorMap mapA, const __gr
         mbar_wait(&tm_full[ts], tph);
         tc_fence_after();
         const uint32_t taddr = tmem_base + ts * kBN + ((uint32_t)(quad * 32) << 16);
-        if (TMA_ST) {
-          if (quad == 0 && lane == 0) bulk_wait_read();         // the copy engine has read this slot's previous tile
-          asm volatile("bar.sync %0, 128;" ::"r"(1 + ts) : "memory");
-        } else {
-          mbar_wait(&st_empty[ts], sph ^ 1);      // slot free (first use passes)
-        }
+        mbar_wait(&st_empty[ts], sph ^ 1);        // slot free (first use passes)
 #pragma unroll
         for (int half = 0; half < 2; ++half) {
           uint32_t hr[4][8];
@@ -699,27 +634,14 @@ corr_build_tc_staged_kernel(const __grid_constant__ CUtensorMap mapA, const __gr
             if (lane == 0) mbar_arrive(&tm_empty[ts]);
           }
           // level 0: the thread's 4 patch rows x 16 columns = four adjacent 4x4 tiles = one 128-byte run
-          if (TMA_ST) {
-            // dense [128 pixels][128 B] box per half, 16-byte chunk c of row r at chunk c ^ (r & 7) (SWIZZLE_128B)
-            unsigned char* sp = smStage + ts * kStageBytes + half * (kBM * 128) + row * 128;
-#pragma unroll
-            for (int t = 0; t < 4 && !(GOSLAM_ST_EXP & 4); ++t) {
-              *reinterpret_cast<uint4*>(sp + (((2 * t) ^ (row & 7)) << 4)) =
-                  make_uint4(hr[0][2 * t], hr[0][2 * t + 1], hr[1][2 * t], hr[1][2 * t + 1]);
-              *reinterpret_cast<uint4*>(sp + (((2 * t + 1) ^ (row & 7)) << 4)) =
-                  make_uint4(hr[2][2 * t], hr[2][2 * t + 1], hr[3][2 * t], hr[3][2 * t + 1]);
-            }
-          } else {
           unsigned char* sp = slot + half * 128;
 #pragma unroll
-          for (int t = 0; t < 4 && !(GOSLAM_ST_EXP & 4); ++t) {
+          for (int t = 0; t < 4; ++t) {
             *reinterpret_cast<uint4*>(sp + t * 32) = make_uint4(hr[0][2 * t], hr[0][2 * t + 1], hr[1][2 * t], hr[1][2 * t + 1]);
             *reinterpret_cast<uint4*>(sp + t * 32 + 16) = make_uint4(hr[2][2 * t], hr[2][2 * t + 1], hr[3][2 * t], hr[3][2 * t + 1]);
           }
-          }
           // pooled levels go to the band pool: wait (once per band) until its previous content has left
           if (!pool_ok) { mbar_wait(band_empty, (band & 1) ^ 1); pool_ok = true; }
-          if (GOSLAM_ST_EXP & 2) { if (hr[0][0] == 0x12345678u) *reinterpret_cast<uint32_t*>(pool2 + row * p2src) = hr[3][7] ^ hr[1][2]; continue; }
           uint32_t l1[2][4];
 #pragma unroll
           for (int cc = 0; cc < 2; ++cc) {
@@ -735,30 +657,14 @@ corr_build_tc_staged_kernel(const __grid_constant__ CUtensorMap mapA, const __gr
           const uint32_t a1 = pack2(pool_pair(l1[0][2], l1[1][2]), pool_pair(l1[0][3], l1[1][3]));
           *reinterpret_cast<uint2*>(pool2 + row * p2src + half * p2row + xb * 8) = make_uint2(a0, a1);
         }
-        if (TMA_ST) {
-          fence_async_smem();                      // this thread's staged bytes become visible to the copy engine
-          asm volatile("bar.sync %0, 128;" ::"r"(1 + ts) : "memory");
-          if (quad == 0 && lane == 0 && !(GOSLAM_ST_EXP & 1)) {
-            const int yb = item % p.n_yb;
-            const int mt = (item / p.n_yb) % p.n_mt;
-            const int n = item / (p.n_yb * p.n_mt);
-            const int n_out = p.out_slot ? __ldg(p.out_slot + n) : n;
-            const unsigned char* sl = smStage + ts * kStageBytes;
-            tma_store_4d(&mapO, sl, xb * 64, 2 * yb, mt * kBM, n_out);                 // rows past h4_0 / pixels past hw
-            tma_store_4d(&mapO, sl + kBM * 128, xb * 64, 2 * yb + 1, mt * kBM, n_out);   // are clipped by the map
-            bulk_commit();
-          }
-        } else {
-          __syncwarp();
-          if (lane == 0) mbar_arrive(&st_full[ts]);
-        }
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&st_full[ts]);
         tph ^= 1; sph ^= 1;
       }
       if (!pool_ok) mbar_wait(band_empty, (band & 1) ^ 1);     // (a group without a tile in this band)
       __syncwarp();
       if (lane == 0) mbar_arrive(band_full);       // this warp's part of the band pool is complete
     }
-    if (TMA_ST && quad == 0 && lane == 0) bulk_wait_read();     // shared memory must outlive the last copies
   } else {
     // ===================== store warps =====================
     // One STG.256 instruction = 8 source pixels x one whole 128-byte run (lane -> pixel lane/4, 32-byte piece lane%4):
@@ -775,9 +681,8 @@ corr_build_tc_staged_kernel(const __grid_constant__ CUtensorMap mapA, const __gr
       const int n_out = p.out_slot ? __ldg(p.out_slot + n) : n;
       const long long pl0 = (long long)n_out * p.hw + mt * kBM;       // plane of the tile's first source pixel
       const int n_src = min(kBM, p.hw - mt * kBM);                    // valid source pixels of this tile
-      for (int xb = 0; xb < (MODE == 1 ? 0 : p.n_xb); ++xb, ++tile) {
+      for (int xb = 0; xb < p.n_xb; ++xb, ++tile) {
         const int s_ = tile & (kTStages - 1);
-        if (MODE == 2 && s_ == 0) continue;        // that tile leaves through the copy engine
         mbar_wait(&st_full[s_], (tile / kTStages) & 1);
         const bool col_ok = xb * 4 + piece < p.w4_0;
 #pragma unroll
@@ -790,7 +695,7 @@ corr_build_tc_staged_kernel(const __grid_constant__ CUtensorMap mapA, const __gr
             va[g] = *reinterpret_cast<const uint4*>(sp);
             vb[g] = *reinterpret_cast<const uint4*>(sp + 16);
           }
-          if (ty < p.h4_0 && col_ok && !(GOSLAM_ST_EXP & 1)) {
+          if (ty < p.h4_0 && col_ok) {
 #pragma unroll
             for (int g = 0; g < 4; ++g) {
               const int sr = swarp * 32 + g * 8 + sub;
@@ -809,7 +714,7 @@ corr_build_tc_staged_kernel(const __grid_constant__ CUtensorMap mapA, const __gr
       // ---- band write-out: levels 1-3, staged byte-for-byte as they go to memory; consecutive lanes take consecutive
       // 32-byte sectors of one source pixel's piece, so a wavefront carries up to 128 B here too
       mbar_wait(band_full, band & 1);
-      if (p.num_levels > 1 && !(GOSLAM_ST_EXP & 1)) {
+      if (p.num_levels > 1) {
         if (yb < p.h4_1) {
           for (int idx = row; idx < n_src * p.w4_1; idx += kStoreWarps * 32) {
             const int sr = idx / p.w4_1, sec = idx - sr * p.w4_1;
@@ -905,52 +810,17 @@ to_kmajor_kernel(const __half* __restrict__ in, __half* __restrict__ out, int hw
   }
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*,
-                                  const cuuint64_t*, const cuuint64_t*, const cuuint32_t*,
-                                  const cuuint32_t*, CUtensorMapInterleave, CUtensorMapSwizzle,
-                                  CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-EncodeTiledFn get_encode_fn() {
-  static EncodeTiledFn fn = nullptr;
-  if (fn) return fn;
-  void* p = nullptr;
-  cudaDriverEntryPointQueryResult q;
-  if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &q) != cudaSuccess ||
-      q != cudaDriverEntryPointSuccess)
-    return nullptr;
-  fn = reinterpret_cast<EncodeTiledFn>(p);
-  return fn;
-}
-
-#ifndef GOSLAM_TC_EXPERIMENT
-#define GOSLAM_TC_EXPERIMENT 0
-#endif
-#ifndef GOSLAM_TC_BULK
-#define GOSLAM_TC_BULK 0
-#endif
-#ifndef GOSLAM_TC_PINGPONG
-#define GOSLAM_TC_PINGPONG 0
-#endif
-#ifndef GOSLAM_TC_STAGED
-#define GOSLAM_TC_STAGED 1       // -DGOSLAM_TC_STAGED=0: always the direct-store kernel (A/B builds)
-#endif
-#ifndef GOSLAM_TC_TMASTORE
-#define GOSLAM_TC_TMASTORE 0     // A/B builds: 1 = level 0 by tensor-map stores, 2 = half of the tiles (see the kernel)
-#endif
 constexpr int kSmemStagedMax = 227 * 1024 - 1024;
-constexpr int kMaxSlots = 1 << 16;   // slot extent of the output tensor map (a bound for clipping only: slots come from out_slot)
 
-// Tensor maps depend only on (base pointer, frame count, h, w): a factor graph builds from the same
-// video-level K-major buffer for its whole life, so the two cuTensorMapEncodeTiled driver calls per launch
-// (~2 us of host time each) are paid once.  Small most-recently-used table, shared by all threads.
-struct MapKey { const void* base; int F, h, w, kind; };
-struct MapSlot { MapKey key; CUtensorMap map; unsigned long long stamp; bool used; };
-constexpr int kMapSlots = 16;
+// Tensor maps depend only on (base pointer, frame count, h, w): a factor graph builds from the same video-level K-major
+// buffer for its whole life, so the two encodes per launch are paid once.
+enum { kMapA = 0, kMapB = 1 };
 
-bool encode_map(EncodeTiledFn enc, const MapKey& k, CUtensorMap* out) {
-  const cuuint64_t hw = (cuuint64_t)k.h * k.w;
-  if (k.kind == 0) {           // A: [F, hw, 128] as (ch, pixel, frame), box 64 ch x 128 pixels
-    cuuint64_t dims[3] = {(cuuint64_t)kD, hw, (cuuint64_t)k.F};
+bool encode_map(GsEncodeTiledFn enc, const GsMapKey& k, CUtensorMap* out) {
+  const int F = k.dims[0], h = k.dims[1], w = k.dims[2];
+  const cuuint64_t hw = (cuuint64_t)h * w;
+  if (k.kind == kMapA) {       // A: [F, hw, 128] as (ch, pixel, frame), box 64 ch x 128 pixels
+    cuuint64_t dims[3] = {(cuuint64_t)kD, hw, (cuuint64_t)F};
     cuuint64_t strides[2] = {(cuuint64_t)kD * 2, hw * kD * 2};
     cuuint32_t box[3] = {(cuuint32_t)kKBox, (cuuint32_t)kBM, 1};
     cuuint32_t es[3] = {1, 1, 1};
@@ -958,21 +828,9 @@ bool encode_map(EncodeTiledFn enc, const MapKey& k, CUtensorMap* out) {
                CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
                CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
   }
-  if (k.kind == 2) {
-    // level 0 of the tiled slot pool, [slot, pixel, h/4, w/4, 16] halves, as (64-half run, tile row, pixel, slot): a box
-    // is one MMA tile's 128-byte run for 128 source pixels.  k.F = number of slots addressable through the map.
-    const cuuint64_t w4 = (cuuint64_t)gs_cdiv(k.w, 4), h4 = (cuuint64_t)gs_cdiv(k.h, 4);
-    cuuint64_t dims[4] = {w4 * 16, h4, hw, (cuuint64_t)k.F};
-    cuuint64_t strides[3] = {w4 * 32, h4 * w4 * 32, hw * h4 * w4 * 32};
-    cuuint32_t box[4] = {64, 1, (cuuint32_t)kBM, 1};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    return enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(k.base), dims, strides, box, es,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
-  }
   // B: (ch, x, y, frame), box 64 ch x 16 x 8: an image patch; rows / columns outside the image read as zero
-  cuuint64_t dims[4] = {(cuuint64_t)kD, (cuuint64_t)k.w, (cuuint64_t)k.h, (cuuint64_t)k.F};
-  cuuint64_t strides[3] = {(cuuint64_t)kD * 2, (cuuint64_t)k.w * kD * 2, hw * kD * 2};
+  cuuint64_t dims[4] = {(cuuint64_t)kD, (cuuint64_t)w, (cuuint64_t)h, (cuuint64_t)F};
+  cuuint64_t strides[3] = {(cuuint64_t)kD * 2, (cuuint64_t)w * kD * 2, hw * kD * 2};
   cuuint32_t box[4] = {(cuuint32_t)kKBox, (cuuint32_t)kPX, (cuuint32_t)kPY, 1};
   cuuint32_t es[4] = {1, 1, 1, 1};
   return enc(out, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, 4, const_cast<void*>(k.base), dims, strides, box, es,
@@ -980,28 +838,14 @@ bool encode_map(EncodeTiledFn enc, const MapKey& k, CUtensorMap* out) {
              CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-bool cached_map(EncodeTiledFn enc, const MapKey& k, CUtensorMap* out) {
-  static MapSlot table[kMapSlots];
-  static unsigned long long clock = 0;
-  static std::mutex mu;
-  std::lock_guard<std::mutex> lock(mu);
-  int victim = -1;
-  for (int i = 0; i < kMapSlots; ++i) {
-    MapSlot& s = table[i];
-    if (s.used && s.key.base == k.base && s.key.F == k.F && s.key.h == k.h && s.key.w == k.w &&
-        s.key.kind == k.kind) {
-      s.stamp = ++clock;
-      *out = s.map;
-      return true;
-    }
-    // victim: a free slot if there is one, else the least recently used
-    if (victim < 0 || (table[victim].used && (!s.used || s.stamp < table[victim].stamp))) victim = i;
-  }
-  MapSlot& v = table[victim];
-  if (!encode_map(enc, k, &v.map)) { v.used = false; return false; }
-  v.key = k; v.used = true; v.stamp = ++clock;
-  *out = v.map;
-  return true;
+GsMapCache g_maps(16, encode_map);
+GsDeviceOnce g_device_once;
+
+cudaError_t device_init(int) {
+  cudaError_t e = cudaFuncSetAttribute(corr_build_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemTC);
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(corr_build_tc_staged_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemStagedMax);
+  return e;
 }
 
 // launch the tensor-core kernel on K-major (pre-scaled) operands: f1t/f2t = [F1|F2, hw, 128]
@@ -1009,11 +853,11 @@ int launch_tc(const __half* f1t, int F1, const __half* f2t, int F2, const int64_
               const int64_t* jj, int rig, const int* out_slot, int tiled, __half* const* levels,
               int num_levels, int N, int h, int w, cudaStream_t st) {
   const int hw = h * w;
-  EncodeTiledFn enc = get_encode_fn();
-  if (!enc) return GOSLAM_ELAUNCH;
   CUtensorMap mapA, mapB;
-  if (!cached_map(enc, MapKey{f1t, F1, h, w, 0}, &mapA) || !cached_map(enc, MapKey{f2t, F2, h, w, 1}, &mapB))
+  if (!g_maps.get(GsMapKey{f1t, kMapA, {F1, h, w}}, &mapA) || !g_maps.get(GsMapKey{f2t, kMapB, {F2, h, w}}, &mapB))
     return GOSLAM_ELAUNCH;
+  const int rc = gs_device_once(g_device_once, device_init);
+  if (rc != GOSLAM_OK) return rc;
   TcParams p{};
   for (int i = 0; i < 4; ++i) p.lvl[i] = i < num_levels ? levels[i] : nullptr;
   p.num_levels = num_levels; p.N = N; p.h = h; p.w = w; p.hw = hw;
@@ -1025,44 +869,10 @@ int launch_tc(const __half* f1t, int F1, const __half* f2t, int F2, const int64_
   p.w4_1 = gs_cdiv(w >> 1, 4); p.h4_1 = gs_cdiv(h >> 1, 4);
   p.pitch2 = (p.n_xb * 16 + 31) / 32 * 32; p.pitch3 = 32;
   p.aligned = (w % 16 == 0 && h % 8 == 0) ? 1 : 0;
-  // Build-time A/B switches (-DGOSLAM_TC_EXPERIMENT=1 ..., tools/ only): the shipped library has them all 0.
-  p.experiment = GOSLAM_TC_EXPERIMENT;
-  // measured 278 us with bulk stores vs 273 us with plain stores on config 2 — the
-  // limit is past the SM (L2 / fabric), so the TMA path is off by default
-  p.bulk = (p.tiled && GOSLAM_TC_BULK) ? 1 : 0;
-  p.pingpong = (p.tiled && GOSLAM_TC_PINGPONG) ? 1 : 0;
-  // per-device: opt-in shared memory + SM count, looked up once per device
-  static int sm_count[64];
-  static std::mutex dev_mu;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64) dev = 0;
-  int sms;
-  {
-    std::lock_guard<std::mutex> lock(dev_mu);
-    if (sm_count[dev] == 0) {
-      if (cudaFuncSetAttribute(corr_build_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               kSmemTC) != cudaSuccess ||
-          cudaFuncSetAttribute(corr_build_tc_staged_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               kSmemStagedMax) != cudaSuccess ||
-          cudaFuncSetAttribute(corr_build_tc_staged_kernel<GOSLAM_TC_TMASTORE ? GOSLAM_TC_TMASTORE : 1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                               kSmemStagedMax) != cudaSuccess)
-        return GOSLAM_ELAUNCH;
-      int n = 148;
-      cudaDeviceGetAttribute(&n, cudaDevAttrMultiProcessorCount, dev);
-      sm_count[dev] = n > 0 ? n : 148;
-    }
-    sms = sm_count[dev];
-  }
+  const int sms = gs_sm_count();
   const int grid = p.n_items < sms ? p.n_items : sms;
-  if (p.tiled && !p.bulk && !p.pingpong && p.experiment != 1 && GOSLAM_TC_STAGED && p.num_levels == 4 &&
-      smem_staged(p.n_xb) <= kSmemStagedMax) {
-    CUtensorMap mapO;
-    if (GOSLAM_TC_TMASTORE && cached_map(enc, MapKey{levels[0], kMaxSlots, h, w, 2}, &mapO)) {
-      corr_build_tc_staged_kernel<GOSLAM_TC_TMASTORE><<<grid, kThreadsST, smem_staged(p.n_xb), st>>>(mapA, mapB, mapO, p, pool_bytes_st(p.n_xb));
-    } else {
-      corr_build_tc_staged_kernel<0><<<grid, kThreadsST, smem_staged(p.n_xb), st>>>(mapA, mapB, mapA, p, pool_bytes_st(p.n_xb));
-    }
+  if (p.tiled && p.num_levels == 4 && smem_staged(p.n_xb) <= kSmemStagedMax) {
+    corr_build_tc_staged_kernel<<<grid, kThreadsST, smem_staged(p.n_xb), st>>>(mapA, mapB, p, pool_bytes_st(p.n_xb));
     GS_CHECK_LAUNCH();
     return GOSLAM_OK;
   }

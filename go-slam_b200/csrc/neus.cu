@@ -21,25 +21,16 @@
 // alpha + embedding), phase 2 is the warp-wide MLP on m16n8k16 tensor-core tiles with the
 // weights resident in shared memory, phase 3 composites each ray with a warp scan.
 #include "common.cuh"
+#include "launch.cuh"
 #include <math.h>
 #include <algorithm>
-#include <mutex>
 
 namespace {
 
 constexpr int kLevels = 16;
 // code-size knobs (the kernel body is ~60 KB of SASS; ncu shows warps starved on instruction fetch)
-#ifndef GOSLAM_NEUS_KUNROLL
-#define GOSLAM_NEUS_KUNROLL 8
-#endif
-#ifndef GOSLAM_NEUS_HUNROLL
-#define GOSLAM_NEUS_HUNROLL 1
-#endif
-constexpr int kNeusKUnroll = GOSLAM_NEUS_KUNROLL, kNeusHUnroll = GOSLAM_NEUS_HUNROLL;
-#ifndef GOSLAM_NEUS_THREADS
-#define GOSLAM_NEUS_THREADS 384
-#endif
-constexpr int kThreadsN = GOSLAM_NEUS_THREADS;
+constexpr int kNeusKUnroll = 8, kNeusHUnroll = 1;
+constexpr int kThreadsN = 384;
 constexpr int kWarpsN = kThreadsN / 32;
 constexpr int kDenseLevels = 5;     // levels whose res^3 fits the table (16,24,34,49,71)
 constexpr int kIn = 80, kInPad = 88;     // MLP input width / padded smem row (halves)
@@ -1175,14 +1166,7 @@ __global__ void __launch_bounds__(kMbWarps * 32, 1) neus_mlp_bwd_kernel(const Ml
 }
 
 // hash-grid constants are per DEVICE (constant memory) and the opt-in shared memory is per device too
-int neus_device_init() {
-  static bool ready[64];
-  static std::mutex mu;
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (dev < 0 || dev >= 64) return GOSLAM_EINVAL;
-  std::lock_guard<std::mutex> lock(mu);
-  if (ready[dev]) return GOSLAM_OK;
+cudaError_t neus_device_setup(int) {
   GridMeta g = make_grid_meta(nullptr);
   LevelConst lc[kLevels];
   for (int l = 0; l < kLevels; ++l) {
@@ -1193,16 +1177,18 @@ int neus_device_init() {
     lc[l].size = g.size[l];
     const unsigned long long dense = (unsigned long long)g.res[l] * g.res[l] * g.res[l];
     const bool hashed = dense > g.size[l];
-    if (hashed != (l >= kDenseLevels) || (hashed && g.size[l] != (1u << 19))) return GOSLAM_EINVAL;
+    if (hashed != (l >= kDenseLevels) || (hashed && g.size[l] != (1u << 19))) return cudaErrorInvalidValue;
   }
-  if (cudaMemcpyToSymbol(c_lvl, lc, sizeof(lc)) != cudaSuccess) return GOSLAM_ELAUNCH;
-  if (cudaFuncSetAttribute(neus_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           (int)sizeof(Smem)) != cudaSuccess) return GOSLAM_ELAUNCH;
-  if (cudaFuncSetAttribute(neus_mlp_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           (int)sizeof(MlpBwdSmem)) != cudaSuccess) return GOSLAM_ELAUNCH;
-  ready[dev] = true;
-  return GOSLAM_OK;
+  cudaError_t e = cudaMemcpyToSymbol(c_lvl, lc, sizeof(lc));
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(neus_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
+  if (e == cudaSuccess)
+    e = cudaFuncSetAttribute(neus_mlp_bwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(MlpBwdSmem));
+  return e;
 }
+
+GsDeviceOnce g_neus_once;
+int neus_device_init() { return gs_device_once(g_neus_once, neus_device_setup); }
 
 }  // namespace
 

@@ -107,19 +107,7 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-// bulk (TMA) copy shared -> global, tracked by the bulk async-group of the issuing thread
-__device__ __forceinline__ void bulk_store(void* gdst, const void* ssrc, uint32_t bytes) {
-  asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(gdst),
-               "r"(smem_u32(ssrc)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void tma_store_4d(const CUtensorMap* map, const void* src, int c0, int c1, int c2, int c3) {
-  asm volatile("cp.async.bulk.tensor.4d.global.shared::cta.bulk_group [%0, {%2, %3, %4, %5}], [%1];" ::"l"(map),
-               "r"(smem_u32(src)), "r"(c0), "r"(c1), "r"(c2), "r"(c3)
-               : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_all() { asm volatile("cp.async.bulk.wait_group 0;" ::: "memory"); }
+// generic-proxy shared-memory writes become visible to the async proxy (tensor core, TMA)
 __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
 
 // K-major, SWIZZLE_128B shared-memory matrix descriptor (cute::UMMA::SmemDescriptor):

@@ -58,7 +58,8 @@ def test_tcgen05_build_vs_oracle(hw):
 
 
 @pytest.mark.parametrize("layout", ["tiled", "rowmajor"])
-@pytest.mark.parametrize("hw,rig", [((48, 64), 1), ((40, 80), 1), ((30, 40), 1), ((40, 60), 2), ((60, 80), 1)])
+@pytest.mark.parametrize("hw,rig", [((48, 64), 1), ((40, 80), 1), ((30, 40), 1), ((40, 60), 2), ((60, 80), 1),
+                                    ((24, 96), 1)])
 def test_pool_build_and_lookup_vs_oracle(hw, rig, layout):
     """FactorGraph's path: video-level K-major maps -> pooled (tiled / row-major) tensor-core build ->
     pooled 4-level lookup; stereo rigs use the right image for self-edges (src/factor_graph.py:108-111)."""
